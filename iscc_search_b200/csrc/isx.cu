@@ -21,6 +21,7 @@
 #include "kernels.cuh"
 #include "keymap.hpp"
 #include "small.cuh"
+#include "tc.cuh"
 
 namespace isx {
 
@@ -176,6 +177,8 @@ struct isx_store {
     PinnedBuf h_small_dbg;
     bool small_ok = true;           // cooperative launch available
     int small_smem_max = -1;        // dynamic shared memory k_scan_small may use on this device (set on first use)
+    // function attributes are per device: the scan kernels whose shared-memory limit this store has raised, bit WE
+    uint32_t scan_attr_done = 0, scan_tc_attr_done = 0;
     // isx_search (host results): the fused select writes straight into the pinned result block (no D2H copies)
     uint64_t* small_host_khi = nullptr; uint64_t* small_host_klo = nullptr; uint16_t* small_host_h = nullptr;
     uint16_t* small_host_n = nullptr; uint32_t* small_host_cnt = nullptr;
@@ -379,10 +382,9 @@ static int launch_scan_t(isx_store* s, ScanParams& p, uint32_t grid_cap_per_sm, 
         p.stage_cap = cap >= 64 ? (uint32_t)cap : 0;
         if (p.stage_cap) smem += stage_bytes(p.stage_cap);
     }
-    static bool attr_done = false;
-    if (!attr_done || smem > 48 * 1024) {
+    if (!(s->scan_attr_done & (1u << WE))) {
         CU(cudaFuncSetAttribute(k_scan<WE, G, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, s->max_smem_optin));
-        attr_done = true;
+        s->scan_attr_done |= 1u << WE;
     }
     uint32_t n_blocks = p.block_end - p.block_begin;
     uint32_t n_groups = (n_blocks + G - 1) / G;
@@ -396,6 +398,61 @@ static int launch_scan_t(isx_store* s, ScanParams& p, uint32_t grid_cap_per_sm, 
     s->stats.kernel_launches++;
     s->stats.scan_launches++;
     return 0;
+}
+
+// ---- tensor-core scan (tc.cuh) ----
+template <int WE>
+static int launch_scan_tc_t(isx_store* s, ScanParams& p, cudaStream_t stream) {
+    size_t smem = tc_smem_bytes(WE, p.q_split, p.R) + 8;   // + alignment of the stage
+    {
+        const size_t per_cta = (size_t)s->smem_per_sm / kTcMinBlocksPerSm - 1024;
+        size_t cap = per_cta > smem + stage_bytes(0) ? (per_cta - smem - stage_bytes(0)) / 12 : 0;
+        cap = std::min<size_t>(cap, 1024) & ~(size_t)31;
+        p.stage_cap = cap >= 64 ? (uint32_t)cap : 0;
+        if (p.stage_cap) smem += stage_bytes(p.stage_cap);
+    }
+    if (!(s->scan_tc_attr_done & (1u << WE))) {
+        CU(cudaFuncSetAttribute(k_scan_tc<WE>, cudaFuncAttributeMaxDynamicSharedMemorySize, s->max_smem_optin));
+        s->scan_tc_attr_done |= 1u << WE;
+    }
+    const uint32_t n_blocks = p.block_end - p.block_begin;
+    if (n_blocks == 0) return 0;
+    const uint32_t gx = std::min<uint32_t>(n_blocks, (uint32_t)s->sm_count * kTcMinBlocksPerSm);
+    dim3 grid(gx, (p.T + p.q_split - 1) / p.q_split, 1);
+    k_scan_tc<WE><<<grid, kThreads, smem, stream>>>(p);
+    CU(cudaGetLastError());
+    s->stats.kernel_launches++;
+    s->stats.scan_launches++;
+    return 0;
+}
+
+// ISX_TC_SCAN=0 keeps every launch on the POPC scan (A/B on the same build); ISX_TC_MIN_T sets the smallest query tile
+// that takes the tensor-core scan (below it the MMA's N would be mostly padding)
+static bool use_tc_scan(uint32_t T) {
+    static const bool env_on = [] { const char* e = getenv("ISX_TC_SCAN"); return !(e && e[0] == '0'); }();
+    static const uint32_t env_min_t = [] { const char* e = getenv("ISX_TC_MIN_T"); return e ? (uint32_t)std::max(1, atoi(e)) : 64u; }();
+    return env_on && T >= env_min_t;
+}
+
+static int launch_scan_tc(isx_store* s, ScanParams& p, uint32_t we, uint32_t bpi_hint, cudaStream_t stream) {
+    p.blocks_per_item = std::max<uint32_t>(1, bpi_hint);
+    // <= 256 queries per CTA (the MMA's N); small ranges split the tile further, down to 64 queries, so ~4 waves of CTAs exist
+    const uint32_t n_blocks = std::max<uint32_t>(1, p.block_end - p.block_begin);
+    const uint32_t want = (uint32_t)s->sm_count * kTcMinBlocksPerSm * 4;
+    uint32_t splits = (p.T + kTcMaxN - 1) / kTcMaxN;
+    if (n_blocks * splits < want) splits = std::max(splits, std::min((want + n_blocks - 1) / n_blocks, std::max<uint32_t>(1, p.T / 64)));
+    p.q_split = (p.T + splits - 1) / splits;
+    switch (we) {
+        case 1: return launch_scan_tc_t<1>(s, p, stream);
+        case 2: return launch_scan_tc_t<2>(s, p, stream);
+        case 3: return launch_scan_tc_t<3>(s, p, stream);
+        case 4: return launch_scan_tc_t<4>(s, p, stream);
+        case 5: return launch_scan_tc_t<5>(s, p, stream);
+        case 6: return launch_scan_tc_t<6>(s, p, stream);
+        case 7: return launch_scan_tc_t<7>(s, p, stream);
+        case 8: return launch_scan_tc_t<8>(s, p, stream);
+    }
+    return fail(ISX_EINVAL, "bad word count %u", we);
 }
 
 static uint32_t groups_for(uint32_t we) { return we <= 2 ? 4 : (we <= 4 ? 2 : 1); }
@@ -453,7 +510,8 @@ static int scan_range(isx_store* s, ScanParams& p, uint32_t b0, uint32_t b1, uin
                 stream = sides[side_used];
                 CU(cudaStreamWaitEvent(stream, fork_ev, 0));
             }
-            int rc = launch_scan(s, p, (m + 3) / 4, bpi_hint, stream);
+            const bool tc = use_tc_scan(p.T);
+            int rc = tc ? launch_scan_tc(s, p, (m + 3) / 4, bpi_hint, stream) : launch_scan(s, p, (m + 3) / 4, bpi_hint, stream);
             if (rc) return rc;
             if (stream != main_stream) {
                 CU(cudaEventRecord(join_ev[side_used], stream));
@@ -474,7 +532,7 @@ static int scan_range(isx_store* s, ScanParams& p, uint32_t b0, uint32_t b1, uin
             s->stats.algo_bytes += rows * m;
             s->stats.algo_popc += rows * p.T * ((m + 3) / 4);
             static const uint32_t kCsaPopc[9] = {0, 1, 1, 2, 2, 3, 2, 3, 3};  // steady state: OR-fold lower-bound filter (3-word folds for 6..8 words, 2-word folds for 2, 4, 5) else carry-save
-            s->stats.issued_popc += rows * p.T * kCsaPopc[(m + 3) / 4];
+            if (!tc) s->stats.issued_popc += rows * p.T * kCsaPopc[(m + 3) / 4];   // the tensor-core scan issues no POPC
         }
         if (Lhi == kMaxBytes) break;
     }
@@ -1840,11 +1898,47 @@ static int selftest_distance_we(uint64_t n, uint64_t& x) {
     return 0;
 }
 
+// Host build of the tensor-core scan's encoding (tc.cuh): rows as 0/1 bytes, queries as +-1 bytes zeroed past 8m bits, the
+// byte dot product acc over the K-major layout, h = acc + popc(q[:m]) against a naive popcount, for every length m 1..32.
+static int selftest_tc_encoding(uint64_t n, uint64_t& x) {
+    auto next = [&]() { x ^= x << 13; x ^= x >> 7; x ^= x << 17; return x; };
+    for (uint64_t it = 0; it < n; it++) {
+        for (uint32_t m = 1; m <= kMaxBytes; m++) {
+            const uint32_t WE = (m + 3) / 4, KB = 32 * WE;
+            uint32_t a[8], q[8];
+            const uint32_t sparse = (uint32_t)(it % 3);   // random rows, near-identical rows, identical rows
+            for (uint32_t w = 0; w < WE; w++) {
+                q[w] = (uint32_t)next();
+                const uint64_t v = next();
+                a[w] = sparse == 0 ? (uint32_t)v : sparse == 1 ? (q[w] ^ (uint32_t)(v & (v >> 16) & (v >> 32))) : q[w];
+            }
+            // row r = 1 and query row 9 of a 16-row tile: the second core matrix row group exercises the layout
+            std::vector<int8_t> A(16 * KB, 0), B(16 * KB, 0);
+            uint32_t popc_q = 0, exact = 0;
+            for (uint32_t w = 0; w < WE; w++) {
+                const uint32_t nb = tc_word_bits(m, w), mk = nb >= 32 ? 0xffffffffu : (1u << nb) - 1u;
+                popc_q += popc32(q[w] & mk);
+                exact += popc32((a[w] ^ q[w]) & mk);
+                for (int j = 0; j < 8; j++) {
+                    const uint32_t ra = tc_row_bytes(a[w], j), qb = tc_query_bytes(q[w], j, nb);
+                    memcpy(&A[tc_off(1, 32 * w + 4 * j, KB)], &ra, 4);
+                    memcpy(&B[tc_off(9, 32 * w + 4 * j, KB)], &qb, 4);
+                }
+            }
+            int32_t acc = 0;
+            for (uint32_t kb = 0; kb < KB; kb++) acc += (int32_t)A[tc_off(1, kb, KB)] * (int32_t)B[tc_off(9, kb, KB)];
+            if (tc_hamming(acc, popc_q) != exact) return fail(ISX_EINVAL, "tensor-core encoding differs from the naive popcount at m = %u", m);
+        }
+    }
+    return 0;
+}
+
 extern "C" {
 
 int isx_selftest_distance(uint64_t n, uint64_t seed) {
     uint64_t x = seed * 0x9E3779B97F4A7C15ull + 1;
     int rc = 0;
+    if ((rc = selftest_tc_encoding(n, x))) return rc;
     if ((rc = selftest_distance_we<1>(n, x)) || (rc = selftest_distance_we<2>(n, x)) || (rc = selftest_distance_we<3>(n, x)) ||
         (rc = selftest_distance_we<4>(n, x)) || (rc = selftest_distance_we<5>(n, x)) || (rc = selftest_distance_we<6>(n, x)) ||
         (rc = selftest_distance_we<7>(n, x)) || (rc = selftest_distance_we<8>(n, x)))

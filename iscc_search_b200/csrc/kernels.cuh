@@ -220,6 +220,18 @@ __device__ __forceinline__ bool stage_direct(const ScanParams& p, uint32_t q, ui
     return ((slot + 1) >> p.tighten_shift) != (slot >> p.tighten_shift);
 }
 
+// one candidate of query q to the stage, by one thread (straight to HBM when the stage is full)
+__device__ __forceinline__ void stage_push(const ScanParams& p, const Stage& st, uint32_t q, uint64_t c) {
+    const uint32_t idx = atomicAdd(&st.counters[0], 1u) - st.counters[1];
+    if (idx < p.stage_cap) {
+        st.cand[idx] = c;
+        st.query[idx] = q;
+    } else if (stage_direct(p, q, c)) {
+        const uint32_t j = atomicAdd(&st.counters[2], 1u) - st.counters[3];
+        if (j < kStagePending) st.pending[j] = q;   // beyond that: the threshold just stays looser for a while
+    }
+}
+
 // entered by the whole warp when any lane has a row of the group within the bound of query q
 __device__ __noinline__ void stage_group(const ScanParams& p, uint32_t q, uint32_t hmax, uint32_t d0, uint32_t d1, uint32_t d2,
                                          uint32_t d3, uint32_t seg, uint32_t row0, uint32_t seg_n, const uint16_t* s_rank) {
@@ -231,17 +243,8 @@ __device__ __noinline__ void stage_group(const ScanParams& p, uint32_t q, uint32
     const uint32_t d[4] = {d0, d1, d2, d3};
 #pragma unroll
     for (int r = 0; r < 4; r++) {
-        if (d[r] <= hmax && row0 + r < seg_n) {   // padding rows of the last block never emit
-            const uint64_t c = pack_cand(s_rank[d[r]], d[r], seg, row0 + r);
-            const uint32_t idx = atomicAdd(&st.counters[0], 1u) - st.counters[1];
-            if (idx < p.stage_cap) {
-                st.cand[idx] = c;
-                st.query[idx] = q;
-            } else if (stage_direct(p, q, c)) {
-                const uint32_t j = atomicAdd(&st.counters[2], 1u) - st.counters[3];
-                if (j < kStagePending) st.pending[j] = q;   // beyond that: the threshold just stays looser for a while
-            }
-        }
+        if (d[r] <= hmax && row0 + r < seg_n)   // padding rows of the last block never emit
+            stage_push(p, st, q, pack_cand(s_rank[d[r]], d[r], seg, row0 + r));
     }
 }
 
