@@ -187,6 +187,27 @@ int isx_match_all(isx_store_t* s, const uint8_t* query, uint32_t qlen, uint32_t 
                   void* keys_out, uint16_t* hamming_out, uint16_t* nbits_out, uint64_t* total_out);
 
 /*
+ * Self-join: every unordered pair {a, b} of two distinct stored rows with h * thr_den <= thr_num * nbits (thr_den != 0),
+ * h = popc(a[:m] ^ b[:m]), m = min(len a, len b) bytes, nbits = 8m - the threshold rule of isx_search (thr_num = 0: exact
+ * duplicates plus prefix-equal rows of different lengths, the INSTANCE semantics). Which codes of the store are
+ * near-duplicates of each other, without k and without a round trip of the codes through the host.
+ * Each pair is scored once on the device and kept there as one record (key_a, key_b, h, nbits) with key_a < key_b
+ * (8-byte keys: uint64 order; 16-byte keys: bytewise), all records in ascending (key_a, key_b) order; *total_out = pairs.
+ * The result does not depend on row placement. It lives in the store's working memory until the next search or match,
+ * add / remove / clear / load, isx_release_scratch or isx_close. Nothing is truncated: when the records do not fit in
+ * device memory the call fails with ISX_ENOMEM, *total_out still set to the number of pairs found.
+ * Takes the same locks as a search; isx_get_stats reports it like a search (scan launches, pairs scored, candidates).
+ */
+int isx_self_join(isx_store_t* s, uint32_t thr_num, uint32_t thr_den, uint64_t* total_out);
+/*
+ * Records [first, first + n) of the last isx_self_join, in (key_a, key_b) order, into host buffers: keys_a_out and
+ * keys_b_out (n x key_bytes, the key form of isx_search), hamming_out, nbits_out. Fetch a large result in pages.
+ * ISX_EINVAL when the result has ended (see above) or the range lies past the join's total.
+ */
+int isx_join_fetch(isx_store_t* s, uint64_t first, size_t n, void* keys_a_out, void* keys_b_out, uint16_t* hamming_out,
+                   uint16_t* nbits_out);
+
+/*
  * Simprint asset scoring on the device (the per-asset loop of iscc_search/indexes/simprint/usearch_core.py:199-269):
  * the best record of every (asset, query simprint) pair, grouped by asset (segment a = records [seg[a], seg[a+1])),
  * ascending query index inside a segment: rec_qi (query index), rec_sim (1 - h/ndim), rec_idf (IDF of the matched

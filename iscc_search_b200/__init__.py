@@ -8,10 +8,10 @@ Public surface:
 All search arithmetic runs in libisx_b200.so (hand-written sm_100a CUDA); there is no CPU path.
 """
 
-from iscc_search_b200.matches import BatchMatches, Match, Matches  # noqa: F401
+from iscc_search_b200.matches import BatchMatches, JoinPairs, Match, Matches  # noqa: F401
 from iscc_search_b200.nphd import MultiDeviceIndex128, MultiDeviceNphdIndex, ShardedIndex128, ShardedNphdIndex  # noqa: F401
 from iscc_search_b200.utils import timer  # noqa: F401
 from iscc_search_b200.backend import B200Index, B200IndexManager  # noqa: F401
 
-__all__ = ["B200IndexManager", "B200Index", "ShardedNphdIndex", "MultiDeviceNphdIndex", "ShardedIndex128", "MultiDeviceIndex128", "Matches", "BatchMatches", "Match", "timer"]
+__all__ = ["B200IndexManager", "B200Index", "ShardedNphdIndex", "MultiDeviceNphdIndex", "ShardedIndex128", "MultiDeviceIndex128", "Matches", "BatchMatches", "Match", "JoinPairs", "timer"]
 __version__ = "0.1.0"

@@ -50,7 +50,7 @@ SYMBOLS = (
     "isx_last_error", "isx_abi_version", "isx_device_count", "isx_open", "isx_close", "isx_set_stream",
     "isx_set_profiling", "isx_get_stats", "isx_add", "isx_add_device", "isx_synth_rows_device", "isx_remove", "isx_contains", "isx_get", "isx_size",
     "isx_clear", "isx_release_scratch", "isx_device_bytes", "isx_length_mask", "isx_save", "isx_load", "isx_search",
-    "isx_search_device", "isx_merge_device", "isx_max_k", "isx_match_all", "isx_score_segments", "isx_share_init", "isx_share_attach",
+    "isx_search_device", "isx_merge_device", "isx_max_k", "isx_match_all", "isx_self_join", "isx_join_fetch", "isx_score_segments", "isx_share_init", "isx_share_attach",
     "isx_share_reset", "isx_share_set_lengths", "isx_selftest_rank_table", "isx_selftest_keymap", "isx_selftest_distance",
 )
 
@@ -58,7 +58,7 @@ SYMBOLS = (
 def build(force=False):
     # type: (bool) -> Path
     """Compile csrc/ for sm_100a with nvcc (in-tree, so the .so ships with the repo snapshot)."""
-    srcs = [CSRC / "isx.cu", CSRC / "kernels.cuh", CSRC / "small.cuh", CSRC / "keymap.hpp", _PKG.parent / "include" / "isx.h"]
+    srcs = [CSRC / "isx.cu", CSRC / "kernels.cuh", CSRC / "small.cuh", CSRC / "tc.cuh", CSRC / "join.cuh", CSRC / "keymap.hpp", _PKG.parent / "include" / "isx.h"]
     stale = not SO_PATH.exists() or any(p.stat().st_mtime > SO_PATH.stat().st_mtime for p in srcs)
     if force or stale:
         r = subprocess.run(["make", "-C", str(CSRC)], capture_output=True, text=True)
@@ -108,6 +108,8 @@ def lib():
     L.isx_merge_device.argtypes = [vp, u32, sz, u32, sz, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, ci]
     L.isx_max_k.argtypes = [vp, P(u32)]
     L.isx_match_all.argtypes = [vp, vp, u32, u32, u32, sz, vp, vp, vp, P(u64)]
+    L.isx_self_join.argtypes = [vp, u32, u32, P(u64)]
+    L.isx_join_fetch.argtypes = [vp, u64, sz, vp, vp, vp, vp]
     L.isx_score_segments.argtypes = [vp, vp, sz, vp, vp, vp, sz, vp, u32, vp]
     L.isx_share_init.argtypes = [vp, u32, u32, u32, vp]
     L.isx_share_attach.argtypes = [vp, u32, vp]
@@ -295,6 +297,35 @@ class Store:
                 n = int(total.value)
                 return keys[:n], h[:n], nb[:n]
             max_out = int(total.value) + 1024
+
+    def self_join(self, thr, page=1 << 22):
+        # type: (tuple[int,int], int) -> tuple
+        """
+        Every pair of stored rows within h/nbits <= thr[0]/thr[1] (include/isx.h: isx_self_join), fetched in pages of
+        `page` records -> (keys_a, keys_b, hamming uint16[n], nbits uint16[n]) with key_a < key_b, ascending (key_a, key_b).
+        Keys have the form of `search`: uint64[n], or uint8[n,16] for 16-byte keys.
+        """
+        total = ctypes.c_uint64()
+        check(lib().isx_self_join(self.handle, thr[0], thr[1], ctypes.byref(total)))
+        n = int(total.value)
+        shape = (n,) if self.key_bytes == 8 else (n, 16)
+        dt = np.uint64 if self.key_bytes == 8 else np.uint8
+        ka, kb = np.zeros(shape, dtype=dt), np.zeros(shape, dtype=dt)
+        h, nb = np.zeros(n, dtype=np.uint16), np.zeros(n, dtype=np.uint16)
+        for i0 in range(0, n, page):
+            c = min(page, n - i0)
+            check(lib().isx_join_fetch(self.handle, i0, c, ptr(ka[i0:]), ptr(kb[i0:]), ptr(h[i0:]), ptr(nb[i0:])))
+        return ka, kb, h, nb
+
+    def join_fetch(self, first, n):
+        # type: (int, int) -> tuple
+        """Records [first, first+n) of the last self_join (include/isx.h: isx_join_fetch)."""
+        shape = (n,) if self.key_bytes == 8 else (n, 16)
+        dt = np.uint64 if self.key_bytes == 8 else np.uint8
+        ka, kb = np.zeros(shape, dtype=dt), np.zeros(shape, dtype=dt)
+        h, nb = np.zeros(n, dtype=np.uint16), np.zeros(n, dtype=np.uint16)
+        check(lib().isx_join_fetch(self.handle, first, n, ptr(ka), ptr(kb), ptr(h), ptr(nb)))
+        return ka, kb, h, nb
 
     def set_stream(self, cuda_stream):
         """

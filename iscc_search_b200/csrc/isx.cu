@@ -19,6 +19,7 @@
 
 #include "../../include/isx.h"
 #include "kernels.cuh"
+#include "join.cuh"
 #include "keymap.hpp"
 #include "small.cuh"
 #include "tc.cuh"
@@ -183,6 +184,13 @@ struct isx_store {
     uint64_t* small_host_khi = nullptr; uint64_t* small_host_klo = nullptr; uint16_t* small_host_h = nullptr;
     uint16_t* small_host_n = nullptr; uint32_t* small_host_cnt = nullptr;
     bool small_host_valid = false, small_host_used = false;
+    // self-join (isx_self_join): the sorted pair records of the last join, in d_join_keys / d_join_vals [join_cur] (the
+    // other buffer of each pair is the sort's scratch); valid until the next search or match, a mutation (version), or
+    // release_scratch
+    DevBuf d_join_keys[2], d_join_vals[2], d_join_tmp, d_join_rows, d_join_cnt;
+    uint32_t join_cur = 0;
+    uint64_t join_total = 0, join_version = 0;
+    bool join_valid = false;
     cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
     std::vector<cudaEvent_t> tile_events;  // 3 per tile, grown on demand (profiling only)
     isx_stats_t stats{};
@@ -708,6 +716,7 @@ static int search_core(isx_store* s, const uint8_t* queries, bool q_on_device, c
                        uint32_t thr_num, uint32_t thr_den, const SearchOut& out) {
     isx_stats_t& st = s->stats;
     st = isx_stats_t{};
+    s->join_valid = false;
     const bool share_armed = s->share_armed;  // consumed by this call whatever happens next
     s->share_armed = false;
     if (Q == 0) return 0;
@@ -1068,6 +1077,224 @@ static int search_core(isx_store* s, const uint8_t* queries, bool q_on_device, c
     return 0;
 }
 
+// ---- self-join (join.cuh, DESIGN.md §3.7) ------------------------------------------------------------------------------
+constexpr uint32_t kJoinCap = 1024;   // candidate list per query of a chunk; a query with more partners is re-scanned exactly
+
+// grow a device buffer to at least `want` bytes, keeping its first `used` bytes; ISX_ENOMEM (no message, the error state
+// cleared) when the device has no room - the caller decides what that means
+static int grow_keep(isx_store* s, DevBuf& b, size_t used, size_t want) {
+    if (want <= b.cap) return 0;
+    void* p = nullptr;
+    size_t bytes = want + want / 4 + 256;
+    cudaError_t e = cudaMalloc(&p, bytes);
+    if (e != cudaSuccess) { cudaGetLastError(); bytes = want; e = cudaMalloc(&p, bytes); }
+    if (e != cudaSuccess) { cudaGetLastError(); return ISX_ENOMEM; }
+    if (used) {
+        e = cudaMemcpyAsync(p, b.p, used, cudaMemcpyDeviceToDevice, s->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(s->stream);
+        if (e != cudaSuccess) { cudaFree(p); return fail(ISX_ECUDA, "self-join: copying the pair records failed: %s", cudaGetErrorString(e)); }
+    }
+    if (b.p) cudaFree(b.p);
+    b.p = p;
+    b.cap = bytes;
+    return 0;
+}
+
+static void release_join(isx_store* s) {
+    for (DevBuf* b : {&s->d_join_keys[0], &s->d_join_keys[1], &s->d_join_vals[0], &s->d_join_vals[1], &s->d_join_tmp}) b->release();
+    s->join_valid = false;
+    s->join_total = 0;
+}
+
+// Every unordered pair of stored rows with h * thr_den <= thr_num * nbits, sorted by (key_a, key_b), left in d_join_*.
+// The live blocks are walked in list order (ascending length, segments in order) in chunks of <= kMaxTile rows of one
+// segment; a chunk's rows become a query tile that is scanned with a fixed threshold against [chunk's first block, end):
+// the rest of its own bucket and every longer bucket. So a pair of different lengths is scored once, from its shorter row,
+// and a pair of one length from its earlier row; k_join_pairs drops what a chunk sees of itself from the other side.
+static int self_join_core(isx_store* s, uint32_t thr_num, uint32_t thr_den, uint64_t* total_out) {
+    isx_stats_t& st = s->stats;
+    st = isx_stats_t{};
+    s->join_valid = false;   // the record buffers of the last join are reused
+    s->join_total = 0;
+    int rc;
+    if ((rc = upload_segs(s)) || (rc = upload_blocks(s))) return rc;
+    const uint32_t n_blocks_total = (uint32_t)s->h_blocks.size();
+    const bool wide = s->key_bytes == 16;
+    const size_t kb = wide ? sizeof(JoinKey16) : sizeof(JoinKey8);
+    uint32_t mask = 0;   // the compared lengths of all pairs are exactly the stored lengths
+    for (uint32_t L = 1; L <= kMaxBytes; L++) if (s->bucket_rows[L]) mask |= 1u << (L - 1);
+    if (n_blocks_total == 0 || s->n_rows < 2) {
+        s->join_valid = true;
+        s->join_version = s->version;
+        return 0;
+    }
+    if ((rc = build_tables(s, mask))) return rc;
+    const RankTables& tb = s->tables;
+    const uint32_t R = tb.R;
+    uint32_t tau = 0;   // largest rank whose fraction is <= thr_num / thr_den
+    while (tau + 1 < R && (uint64_t)tb.frac_h[tau + 1] * thr_den <= (uint64_t)thr_num * tb.frac_n[tau + 1]) tau++;
+    const uint32_t TM = kMaxTile, C = kJoinCap;
+    if (s->d_queries.ensure((size_t)TM * 32) || s->d_tau.ensure((size_t)TM * 4) || s->d_hist.ensure((size_t)TM * R * 4) ||
+        s->d_cnt.ensure((size_t)TM * 4) || s->d_ovf.ensure((size_t)TM * 4) || s->d_cand.ensure((size_t)TM * C * 8) ||
+        s->d_join_rows.ensure((size_t)TM * 4) || s->d_join_cnt.ensure(8) || s->h_flags.ensure((size_t)TM * 4 + 16) ||
+        s->h_qmap.ensure((size_t)TM * 4))
+        return ISX_ENOMEM;
+    CU(cudaMemsetAsync(s->d_join_cnt.p, 0, 8, s->stream));
+    uint32_t* h_cnt = s->h_flags.as<uint32_t>();
+    unsigned long long* h_pairs = reinterpret_cast<unsigned long long*>(s->h_flags.as<uint8_t>() + (size_t)TM * 4);
+    uint64_t cap = std::min<uint64_t>(s->d_join_keys[0].cap / kb, s->d_join_vals[0].cap / 4);   // pair records the output holds
+    bool counting_only = false;   // the device had no room for more records: the join only counts from here on
+
+    // scan a tile of T rows of segment `seg` (rows row0.. or the device list d_rows) against [b0, end); on return the
+    // exact candidate counts are in h_cnt and the records appended so far in *h_pairs
+    auto scan_tile = [&](uint32_t seg, uint32_t row0, const uint32_t* d_rows, uint32_t T, uint32_t b0, uint32_t Ct) -> int {
+        k_rows_as_queries<<<(T * 8 + 255) / 256, 256, 0, s->stream>>>(s->d_segs.as<SegDesc>(), seg, row0, d_rows, T, s->d_queries.as<uint32_t>());
+        CU(cudaGetLastError());
+        k_init_queries<<<std::max<uint32_t>(1, std::min<uint32_t>((T * R + 255) / 256, (uint32_t)s->sm_count * 8)), 256, 0, s->stream>>>(
+            s->d_tau.as<uint32_t>(), s->d_hist.as<uint32_t>(), nullptr, s->d_cnt.as<uint32_t>(), s->d_ovf.as<uint32_t>(), T, R, tau);
+        CU(cudaGetLastError());
+        st.kernel_launches += 2;
+        ScanParams p{};
+        p.segs = s->d_segs.as<SegDesc>();
+        p.blocks = s->d_blocks.as<uint2>();
+        p.queries = s->d_queries.as<uint32_t>();
+        p.T = T;
+        p.qlen_bytes = s->segs[seg].len_bytes;
+        p.tau = s->d_tau.as<uint32_t>();
+        p.hist = s->d_hist.as<uint32_t>();
+        p.cand_cnt = s->d_cnt.as<uint32_t>();
+        p.cand = s->d_cand.as<uint64_t>();
+        p.overflow = s->d_ovf.as<uint32_t>();
+        p.C = Ct; p.R = R; p.k = 1;
+        p.rank_tab = tb.d_rank.as<uint16_t>();
+        p.hmax_tab = tb.d_hmax.as<uint16_t>();
+        p.update_tau = 0;   // fixed threshold: every row within it is emitted
+        if (s->profiling) CU(cudaEventRecord(s->ev[1], s->stream));
+        int rc2 = scan_range(s, p, b0, n_blocks_total, T >= 64 ? 4 : 16);
+        if (rc2) return rc2;
+        if (s->profiling) CU(cudaEventRecord(s->ev[2], s->stream));
+        CU(cudaMemcpyAsync(h_cnt, p.cand_cnt, (size_t)T * 4, cudaMemcpyDeviceToHost, s->stream));
+        CU(cudaMemcpyAsync(h_pairs, s->d_join_cnt.p, 8, cudaMemcpyDeviceToHost, s->stream));
+        CU(cudaStreamSynchronize(s->stream));
+        if (s->profiling) {
+            float t = 0;
+            CU(cudaEventElapsedTime(&t, s->ev[1], s->ev[2]));
+            st.scan_ms += t;
+        }
+        return 0;
+    };
+    // candidate lists of the tile just scanned -> pair records; `bound` >= the records it can append
+    auto append = [&](uint32_t seg, uint32_t row0, const uint32_t* d_rows, uint32_t T, uint32_t Ct, uint64_t bound) -> int {
+        const uint64_t have = *h_pairs, need = have + bound;
+        if (!counting_only && need > cap) {
+            const uint64_t used = std::min(have, cap);
+            int rc2 = grow_keep(s, s->d_join_keys[0], used * kb, need * kb);
+            if (!rc2) rc2 = grow_keep(s, s->d_join_vals[0], used * 4, need * 4);
+            if (rc2 && rc2 != ISX_ENOMEM) return rc2;
+            counting_only = rc2 == ISX_ENOMEM;
+            cap = std::min<uint64_t>(s->d_join_keys[0].cap / kb, s->d_join_vals[0].cap / 4);
+        }
+        JoinParams jp{};
+        jp.segs = s->d_segs.as<SegDesc>();
+        jp.cand = s->d_cand.as<uint64_t>();
+        jp.cand_cnt = s->d_cnt.as<uint32_t>();
+        jp.C = Ct; jp.T = T; jp.seg = seg; jp.row0 = row0; jp.rows = d_rows;
+        jp.counter = s->d_join_cnt.as<unsigned long long>();
+        jp.cap = cap;
+        jp.vals = s->d_join_vals[0].as<uint32_t>();
+        const unsigned grid = (T * 32 + 255) / 256;
+        if (wide) k_join_pairs<JoinKey16><<<grid, 256, 0, s->stream>>>(jp, s->d_join_keys[0].as<JoinKey16>());
+        else k_join_pairs<JoinKey8><<<grid, 256, 0, s->stream>>>(jp, s->d_join_keys[0].as<JoinKey8>());
+        CU(cudaGetLastError());
+        st.kernel_launches++;
+        return 0;
+    };
+
+    std::vector<uint32_t> ovf_rows, ovf_cnt;
+    for (uint32_t b0 = 0; b0 < n_blocks_total; b0++) {
+        const uint32_t seg = s->h_blocks[b0].x, row0 = s->h_blocks[b0].y;
+        if (row0 % TM) continue;   // chunks start every kMaxTile rows of a segment (two blocks; capacities are multiples of 4096)
+        const uint32_t T = std::min<uint32_t>(TM, s->segs[seg].desc.n - row0);
+        st.passes++;
+        if ((rc = scan_tile(seg, row0, nullptr, T, b0, C))) return rc;
+        uint64_t bound = 0;
+        ovf_rows.clear();
+        ovf_cnt.clear();
+        for (uint32_t i = 0; i < T; i++) {
+            st.candidates += h_cnt[i];
+            if (h_cnt[i] <= C) bound += h_cnt[i];
+            else { ovf_rows.push_back(row0 + i); ovf_cnt.push_back(h_cnt[i]); }
+        }
+        if ((rc = append(seg, row0, nullptr, T, C, bound))) return rc;
+        // queries whose list overflowed: re-scanned together, with C = their largest count (so nothing overflows again),
+        // in as few tiles as a 1 GB candidate budget allows
+        st.fallback_queries += ovf_rows.size();
+        for (size_t i0 = 0; i0 < ovf_rows.size();) {
+            size_t i1 = i0;
+            uint32_t Ct = 0;
+            while (i1 < ovf_rows.size()) {
+                const uint32_t c = std::max(Ct, ovf_cnt[i1]);
+                if (i1 > i0 && (uint64_t)(i1 - i0 + 1) * c * 8 > ((uint64_t)1 << 30)) break;
+                Ct = c;
+                i1++;
+            }
+            const uint32_t To = (uint32_t)(i1 - i0);
+            if (s->d_cand.ensure((size_t)To * Ct * 8)) return ISX_ENOMEM;
+            memcpy(s->h_qmap.p, ovf_rows.data() + i0, (size_t)To * 4);
+            CU(cudaMemcpyAsync(s->d_join_rows.p, s->h_qmap.p, (size_t)To * 4, cudaMemcpyHostToDevice, s->stream));
+            if ((rc = scan_tile(seg, 0, s->d_join_rows.as<uint32_t>(), To, b0, Ct))) return rc;
+            uint64_t bound2 = 0;
+            for (uint32_t i = 0; i < To; i++) {
+                if (h_cnt[i] != ovf_cnt[i0 + i])
+                    return fail(ISX_ECUDA, "self-join: the re-scan of an overflowed row found %u partners, the first scan %u", h_cnt[i], ovf_cnt[i0 + i]);
+                bound2 += h_cnt[i];
+            }
+            if ((rc = append(seg, 0, s->d_join_rows.as<uint32_t>(), To, Ct, bound2))) return rc;
+            i0 = i1;
+        }
+    }
+    CU(cudaMemcpyAsync(h_pairs, s->d_join_cnt.p, 8, cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaStreamSynchronize(s->stream));
+    const uint64_t total = *h_pairs;
+    *total_out = total;
+    const size_t per_pair = 2 * (kb + 4);
+    auto no_room = [&]() {
+        release_join(s);
+        return fail(ISX_ENOMEM, "self-join found %llu pairs; they do not fit in device memory (%zu bytes per pair with the sort)",
+                    (unsigned long long)total, per_pair);
+    };
+    if (counting_only || total > cap) return no_room();
+    if (total > 1) {   // sort by (key_a, key_b) on the device: LSD radix passes over the key words
+        if (grow_keep(s, s->d_join_keys[1], 0, total * kb) || grow_keep(s, s->d_join_vals[1], 0, total * 4)) return no_room();
+        size_t tmp_bytes = 0;
+        cudaError_t e;
+        if (wide) {
+            cub::DoubleBuffer<JoinKey16> dk(s->d_join_keys[0].as<JoinKey16>(), s->d_join_keys[1].as<JoinKey16>());
+            cub::DoubleBuffer<uint32_t> dv(s->d_join_vals[0].as<uint32_t>(), s->d_join_vals[1].as<uint32_t>());
+            CU(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, dk, dv, total, JoinKey16Bits{}, s->stream));
+            if (grow_keep(s, s->d_join_tmp, 0, tmp_bytes)) return no_room();
+            e = cub::DeviceRadixSort::SortPairs(s->d_join_tmp.p, tmp_bytes, dk, dv, total, JoinKey16Bits{}, s->stream);
+            s->join_cur = (uint32_t)dk.selector;
+        } else {
+            cub::DoubleBuffer<JoinKey8> dk(s->d_join_keys[0].as<JoinKey8>(), s->d_join_keys[1].as<JoinKey8>());
+            cub::DoubleBuffer<uint32_t> dv(s->d_join_vals[0].as<uint32_t>(), s->d_join_vals[1].as<uint32_t>());
+            CU(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, dk, dv, total, JoinKey8Bits{}, s->stream));
+            if (grow_keep(s, s->d_join_tmp, 0, tmp_bytes)) return no_room();
+            e = cub::DeviceRadixSort::SortPairs(s->d_join_tmp.p, tmp_bytes, dk, dv, total, JoinKey8Bits{}, s->stream);
+            s->join_cur = (uint32_t)dk.selector;
+        }
+        CU(e);
+        CU(cudaStreamSynchronize(s->stream));
+        st.kernel_launches++;   // the sort counts as one step (CUB launches several kernels)
+    } else {
+        s->join_cur = 0;
+    }
+    s->join_total = total;
+    s->join_version = s->version;
+    s->join_valid = true;
+    return 0;
+}
+
 }  // namespace isx
 
 // =================================================================================================
@@ -1163,7 +1390,9 @@ int isx_close(isx_store_t* s) {
     DevBuf* bufs[] = {&s->d_segs, &s->d_blocks, &s->tables.d_rank, &s->tables.d_hmax, &s->d_stage_codes, &s->d_stage_keys,
                       &s->d_stage_dest, &s->d_moves, &s->d_queries, &s->d_tau, &s->d_hist, &s->d_shist, &s->d_cnt, &s->d_ovf, &s->d_cand,
                       &s->d_qmap, &s->d_fb, &s->d_fb_cand, &s->d_out_khi, &s->d_out_klo, &s->d_out_h, &s->d_out_n,
-                      &s->d_out_cnt, &s->d_out_codes, &s->d_bigsort, &s->d_bdesc, &s->d_bulk, &s->d_small};
+                      &s->d_out_cnt, &s->d_out_codes, &s->d_bigsort, &s->d_bdesc, &s->d_bulk, &s->d_small,
+                      &s->d_join_keys[0], &s->d_join_keys[1], &s->d_join_vals[0], &s->d_join_vals[1], &s->d_join_tmp,
+                      &s->d_join_rows, &s->d_join_cnt};
     for (DevBuf* b : bufs) b->release();
     PinnedBuf* pbufs[] = {&s->h_queries, &s->h_qmap, &s->h_flags, &s->h_out, &s->h_small_info, &s->h_small_dbg};
     for (PinnedBuf* b : pbufs) b->release();
@@ -1197,7 +1426,9 @@ int isx_release_scratch(isx_store_t* s, uint64_t* bytes_freed) {
     // demand; rows, keys, descriptors, rank tables and the small-batch state stay
     DevBuf* bufs[] = {&s->d_stage_codes, &s->d_stage_keys, &s->d_stage_dest, &s->d_moves, &s->d_queries, &s->d_tau, &s->d_hist, &s->d_shist,
                       &s->d_cnt, &s->d_ovf, &s->d_cand, &s->d_qmap, &s->d_fb, &s->d_fb_cand, &s->d_out_khi, &s->d_out_klo, &s->d_out_h,
-                      &s->d_out_n, &s->d_out_cnt, &s->d_out_codes, &s->d_bigsort, &s->d_bulk};
+                      &s->d_out_n, &s->d_out_cnt, &s->d_out_codes, &s->d_bigsort, &s->d_bulk, &s->d_join_keys[0], &s->d_join_keys[1],
+                      &s->d_join_vals[0], &s->d_join_vals[1], &s->d_join_tmp, &s->d_join_rows, &s->d_join_cnt};
+    s->join_valid = false;   // the self-join result lives in this working memory
     uint64_t freed = 0;
     for (DevBuf* b : bufs) { freed += b->cap; b->release(); }
     if (bytes_freed) *bytes_freed = freed;
@@ -1694,6 +1925,7 @@ int isx_match_all(isx_store_t* s, const uint8_t* query, uint32_t qlen, uint32_t 
     if (rc) return rc;
     isx_stats_t& st = s->stats;
     st = isx_stats_t{};
+    s->join_valid = false;
     *total_out = 0;
     if ((rc = upload_segs(s)) || (rc = upload_blocks(s))) return rc;
     const uint32_t n_blocks_total = (uint32_t)s->h_blocks.size();
@@ -1753,6 +1985,64 @@ int isx_match_all(isx_store_t* s, const uint8_t* query, uint32_t qlen, uint32_t 
     CU(cudaStreamSynchronize(s->stream));
     if (s->key_bytes == 8) memcpy(keys_out, khi.data(), (size_t)n * 8);
     else for (uint32_t i = 0; i < n; i++) store_key(s, keys_out, i, khi[i], klo[i]);
+    return 0;
+}
+
+int isx_self_join(isx_store_t* s, uint32_t thr_num, uint32_t thr_den, uint64_t* total_out) {
+    if (!s || !total_out) return fail(ISX_EINVAL, "NULL argument");
+    *total_out = 0;
+    if (thr_den == 0) return fail(ISX_EINVAL, "isx_self_join needs a threshold (thr_den != 0)");
+    std::shared_lock<std::shared_mutex> g(s->rows_mu);
+    std::lock_guard<std::mutex> gw(s->work_mu);
+    int rc = set_device(s);
+    if (rc) return rc;
+    if (s->profiling) CU(cudaEventRecord(s->ev[0], s->stream));
+    if ((rc = self_join_core(s, thr_num, thr_den, total_out))) return rc;
+    if (s->profiling) {
+        CU(cudaEventRecord(s->ev[3], s->stream));
+        CU(cudaStreamSynchronize(s->stream));
+        float t = 0;
+        CU(cudaEventElapsedTime(&t, s->ev[0], s->ev[3]));
+        s->stats.total_ms = t;
+    }
+    return 0;
+}
+
+int isx_join_fetch(isx_store_t* s, uint64_t first, size_t n, void* keys_a_out, void* keys_b_out, uint16_t* hamming_out, uint16_t* nbits_out) {
+    if (!s) return fail(ISX_EINVAL, "store is NULL");
+    if (n && (!keys_a_out || !keys_b_out || !hamming_out || !nbits_out)) return fail(ISX_EINVAL, "NULL argument");
+    std::shared_lock<std::shared_mutex> g(s->rows_mu);
+    std::lock_guard<std::mutex> gw(s->work_mu);
+    if (!s->join_valid || s->join_version != s->version)
+        return fail(ISX_EINVAL, "isx_join_fetch: no self-join result (a search, match, mutation or isx_release_scratch since the last "
+                                "isx_self_join ended it; run the join again)");
+    if (first > s->join_total || n > s->join_total - first)
+        return fail(ISX_EINVAL, "isx_join_fetch: records [%llu, %llu) are outside the %llu pairs of the join", (unsigned long long)first,
+                    (unsigned long long)(first + n), (unsigned long long)s->join_total);
+    if (n == 0) return 0;
+    int rc = set_device(s);
+    if (rc) return rc;
+    const bool wide = s->key_bytes == 16;
+    const size_t kb = wide ? sizeof(JoinKey16) : sizeof(JoinKey8);
+    if (s->h_out.ensure(n * (kb + 4))) return ISX_ENOMEM;
+    uint8_t* hk = s->h_out.as<uint8_t>();
+    uint32_t* hv = reinterpret_cast<uint32_t*>(hk + n * kb);
+    CU(cudaMemcpyAsync(hk, s->d_join_keys[s->join_cur].as<uint8_t>() + first * kb, n * kb, cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaMemcpyAsync(hv, s->d_join_vals[s->join_cur].as<uint32_t>() + first, n * 4, cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaStreamSynchronize(s->stream));
+    if (wide) {
+        const JoinKey16* k = reinterpret_cast<const JoinKey16*>(hk);
+        for (size_t i = 0; i < n; i++) {
+            store_key(s, keys_a_out, i, k[i].a_hi, k[i].a_lo);
+            store_key(s, keys_b_out, i, k[i].b_hi, k[i].b_lo);
+        }
+    } else {
+        const JoinKey8* k = reinterpret_cast<const JoinKey8*>(hk);
+        uint64_t* a = reinterpret_cast<uint64_t*>(keys_a_out);
+        uint64_t* b = reinterpret_cast<uint64_t*>(keys_b_out);
+        for (size_t i = 0; i < n; i++) { a[i] = k[i].a; b[i] = k[i].b; }
+    }
+    for (size_t i = 0; i < n; i++) { hamming_out[i] = (uint16_t)(hv[i] & 0xffffu); nbits_out[i] = (uint16_t)(hv[i] >> 16); }
     return 0;
 }
 

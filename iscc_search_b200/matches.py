@@ -89,3 +89,24 @@ class BatchMatches:
 
     def __repr__(self):
         return f"usearch.BatchMatches({int(np.sum(self.counts))} across {len(self)} queries)"
+
+
+@dataclass
+class JoinPairs:
+    """
+    Result of a self-join (`ShardedNphdIndex.self_join`, `ShardedIndex128.self_join`): every pair of stored rows within a
+    threshold, once, as (keys_a[i], keys_b[i]) with keys_a[i] < keys_b[i], in ascending (key_a, key_b) order.
+    Keys have the form of the index's search results (uint64[n], or uint8[n,16] for 128-bit keys).
+    """
+
+    keys_a: np.ndarray
+    keys_b: np.ndarray
+    hamming: np.ndarray  # uint16[n]
+    nbits: np.ndarray  # uint16[n]: 8 * the shorter code's length in bytes
+    distances: np.ndarray  # float32[n], the float `search` returns for the same pair
+
+    def __len__(self):
+        return len(self.hamming)
+
+    def __repr__(self):
+        return f"JoinPairs({len(self)})"

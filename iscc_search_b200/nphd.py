@@ -13,12 +13,13 @@ NPHD distance = float32(h) / float32(nbits) (index.py:2041-2043 reads `float(dis
 Hamming distance = float32(h) (tests/test_usearch_search.py:122-167).
 """
 
+from fractions import Fraction
 from pathlib import Path
 
 import numpy as np
 
 from iscc_search_b200._lib import Store
-from iscc_search_b200.matches import BatchMatches, Matches
+from iscc_search_b200.matches import BatchMatches, JoinPairs, Matches
 
 MAX_BYTES = 32
 SNAPSHOT_NAME = "store.isx"
@@ -69,6 +70,27 @@ def _pack_vectors(vectors, n_expected=None, fixed_len=0, max_bytes=MAX_BYTES):
     if n_expected is not None and n != n_expected:
         raise ValueError(f"number of keys ({n_expected}) and vectors ({n}) differ")
     return codes, lens
+
+
+def _rational_threshold(threshold):
+    # type: (object) -> tuple[int, int]
+    """Fraction | (num, den) of non-negative ints below 2**32 -> (num, den). A float is refused."""
+    if isinstance(threshold, (float, np.floating)):
+        raise ValueError(
+            "self_join needs an exact rational threshold (fractions.Fraction or a (num, den) pair): a float is not one "
+            "rational cut, since h/nbits for different code lengths falls on different sides of its rounded value"
+        )
+    if isinstance(threshold, Fraction):
+        num, den = threshold.numerator, threshold.denominator
+    elif isinstance(threshold, tuple) and len(threshold) == 2 and all(
+        isinstance(v, (int, np.integer)) and not isinstance(v, bool) for v in threshold
+    ):
+        num, den = int(threshold[0]), int(threshold[1])
+    else:
+        raise ValueError("threshold must be a fractions.Fraction or a (num, den) pair of ints")
+    if not (0 <= num < 2**32 and 0 < den < 2**32):
+        raise ValueError(f"threshold {num}/{den}: num and den must be non-negative ints below 2**32, den > 0")
+    return num, den
 
 
 class _IndexBase:
@@ -235,6 +257,23 @@ class ShardedNphdIndex(_IndexBase):
         return BatchMatches(keys=keys, distances=dist, counts=counts.astype(np.int64), hamming=h, nbits=nb,
                             visited_members=n_rows * len(qlens), computed_distances=n_rows * len(qlens))
 
+    def self_join(self, threshold):
+        # type: (Fraction|tuple[int, int]) -> JoinPairs
+        """
+        Every pair of stored codes that are near-duplicates of each other: NPHD h/nbits <= threshold, with
+        nbits = 8 * the shorter code's length in bytes, as an exact rational rule (the one `search` thresholds use).
+        `threshold` is a `fractions.Fraction` or a `(num, den)` pair of non-negative ints below 2**32; a float raises
+        ValueError. `Fraction(0)` gives exact duplicates plus codes that are a prefix of a longer stored code.
+
+        Each pair comes back once with key_a < key_b, in ascending (key_a, key_b) order; `distances` are the float32
+        values `search` returns for the same pair. All pairs are computed on the GPU and returned in full (MemoryError
+        when they do not fit in device memory). This is not usearch's `Index.join`, which computes a one-to-one
+        matching between two indexes.
+        """
+        ka, kb, h, nb = self._store.self_join(_rational_threshold(threshold))
+        dist = (h.astype(np.float32) / np.maximum(nb, 1).astype(np.float32)).astype(np.float32)
+        return JoinPairs(keys_a=ka, keys_b=kb, hamming=h, nbits=nb, distances=dist)
+
 
 class ShardedIndex128(_IndexBase):
     """
@@ -345,6 +384,23 @@ class ShardedIndex128(_IndexBase):
                            visited_members=n_rows, computed_distances=n_rows)
         return BatchMatches(keys=keys, distances=dist, counts=counts.astype(np.int64), hamming=h, nbits=nb, vectors=vec, first=first,
                             visited_members=n_rows * len(qlens), computed_distances=n_rows * len(qlens))
+
+    def self_join(self, threshold_bits):
+        # type: (int) -> JoinPairs
+        """
+        Every pair of stored vectors within `threshold_bits` (0..ndim) Hamming bits of each other (0: exact duplicates).
+        Each pair comes back once with key_a < key_b (16-byte keys compared bytewise), in ascending (key_a, key_b)
+        order; keys are uint8[n,16] like `search` results and `distances` are float32(h). Computed on the GPU and
+        returned in full (MemoryError when the pairs do not fit in device memory). This is not usearch's `Index.join`,
+        which computes a one-to-one matching between two indexes.
+        """
+        if isinstance(threshold_bits, bool) or not isinstance(threshold_bits, (int, np.integer)):
+            raise ValueError("threshold_bits must be an int")
+        t = int(threshold_bits)
+        if not 0 <= t <= self.ndim:
+            raise ValueError(f"threshold_bits must be in 0..{self.ndim}, got {t}")
+        ka, kb, h, nb = self._store.self_join((t, self.ndim))
+        return JoinPairs(keys_a=ka, keys_b=kb, hamming=h, nbits=nb, distances=h.astype(np.float32))
 
 
 class _MultiScratch:
