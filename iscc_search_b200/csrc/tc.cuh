@@ -62,6 +62,7 @@ __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
 // 32 consecutive accumulator columns of this thread's TMEM lane; the wait is tied to the registers so no use moves above it
+// (the micro-benchmark's 32-bit reference for tmem_ld32_pack16)
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
     asm volatile("tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
                  "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
@@ -75,6 +76,22 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
                    "+r"(v[8]), "+r"(v[9]), "+r"(v[10]), "+r"(v[11]), "+r"(v[12]), "+r"(v[13]), "+r"(v[14]), "+r"(v[15]),
                    "+r"(v[16]), "+r"(v[17]), "+r"(v[18]), "+r"(v[19]), "+r"(v[20]), "+r"(v[21]), "+r"(v[22]), "+r"(v[23]),
                    "+r"(v[24]), "+r"(v[25]), "+r"(v[26]), "+r"(v[27]), "+r"(v[28]), "+r"(v[29]), "+r"(v[30]), "+r"(v[31])
+                 :: "memory");
+}
+// the same 32 columns as 16-bit values, two per register: v[i] holds the low 16 bits of column 2i in its low half and of
+// column 2i + 1 in its high half. Asynchronous: no use of v before tmem_wait_ld(v). The memory clobber keeps the load
+// where it is issued, ahead of the shared-memory reads of the compare it is meant to overlap.
+__device__ __forceinline__ void tmem_ld32_pack16(uint32_t taddr, uint32_t (&v)[16]) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.pack::16b.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
+                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
+                   "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
+                 : "r"(taddr) : "memory");
+}
+// waits for every TMEM load this thread issued; tied to v so that no use of v moves above it
+__device__ __forceinline__ void tmem_wait_ld(uint32_t (&v)[16]) {
+    asm volatile("tcgen05.wait::ld.sync.aligned;"
+                 : "+r"(v[0]), "+r"(v[1]), "+r"(v[2]), "+r"(v[3]), "+r"(v[4]), "+r"(v[5]), "+r"(v[6]), "+r"(v[7]),
+                   "+r"(v[8]), "+r"(v[9]), "+r"(v[10]), "+r"(v[11]), "+r"(v[12]), "+r"(v[13]), "+r"(v[14]), "+r"(v[15])
                  :: "memory");
 }
 __device__ __forceinline__ uint32_t ld_nc_u32(const uint32_t* p) {
@@ -99,11 +116,62 @@ __device__ __noinline__ void tc_emit(const ScanParams& p, uint32_t q, uint32_t h
     else stage_direct(p, q, rec);   // no room for a stage: straight to HBM
 }
 
+// The compare epilogue of one tile for one thread: its TMEM lane (taddr: lane << 16, column 0), 32-column chunks
+// c = c0, c0 + 2, ... < nc. s_nt holds -t_q as s16, two columns per u32 in the order of tmem_ld32_pack16, so one
+// VIADDMNMX.S16x2 takes min(m, acc - t_q) of two pairs; four independent minima per chunk, and the load of the warp's next
+// chunk is in flight while a chunk is compared. on_pass(c, v) runs in the live lanes with acc <= t_q in some column of
+// chunk c, after every TMEM load of the thread has completed.
+// No 16-bit sum wraps: |acc| <= 256 (at most 256 compared bits), |t_q| <= 256 (0 <= hmax <= 8m and 0 <= popc(q) <= 8m,
+// m <= 32), and padding columns (acc = 0) hold -t = 0x4000.
+template <typename OnPass>
+__device__ __forceinline__ void tc_compare_tile(uint32_t taddr, uint32_t c0, uint32_t nc, const uint32_t* s_nt, bool live,
+                                                OnPass&& on_pass) {
+    uint32_t va[16], vb[16];
+    auto compare = [&](uint32_t c, uint32_t (&cur)[16], uint32_t (&nxt)[16], bool next_in_flight) {
+        const uint4* nt = reinterpret_cast<const uint4*>(s_nt + c * 16);
+        uint32_t m0 = 0x7fff7fffu, m1 = 0x7fff7fffu, m2 = 0x7fff7fffu, m3 = 0x7fff7fffu;
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            const uint4 t = nt[j];
+            m0 = __viaddmin_s16x2(cur[4 * j], t.x, m0);
+            m1 = __viaddmin_s16x2(cur[4 * j + 1], t.y, m1);
+            m2 = __viaddmin_s16x2(cur[4 * j + 2], t.z, m2);
+            m3 = __viaddmin_s16x2(cur[4 * j + 3], t.w, m3);
+        }
+        const uint32_t mn = __vimin3_s16x2(m0, m1, __vmins2(m2, m3));
+        const bool hit = live && min((int32_t)(int16_t)mn, (int32_t)mn >> 16) <= 0;
+        if (__any_sync(0xffffffffu, hit)) {   // rare
+            if (next_in_flight) tmem_wait_ld(nxt);   // warp-uniform; no call is made with a TMEM load in flight
+            if (hit) on_pass(c, cur);
+        }
+    };
+    if (c0 >= nc) return;
+    tmem_ld32_pack16(taddr + c0 * 32, va);
+    tmem_wait_ld(va);
+    // Two chunks per iteration, so that the buffers swap without copies. The __syncwarp() after each load keeps it where
+    // it is: without it ptxas schedules the load after the compare it should overlap, next to the vote.
+    for (uint32_t c = c0;; c += 4) {
+        const bool b_next = c + 2 < nc;
+        if (b_next) tmem_ld32_pack16(taddr + (c + 2) * 32, vb);
+        __syncwarp();
+        compare(c, va, vb, b_next);
+        if (!b_next) return;
+        tmem_wait_ld(vb);
+        const bool a_next = c + 4 < nc;
+        if (a_next) tmem_ld32_pack16(taddr + (c + 4) * 32, va);
+        __syncwarp();
+        compare(c + 2, vb, va, a_next);
+        if (!a_next) return;
+        tmem_wait_ld(va);
+    }
+}
+
 // WE: words compared per pair (1..8). One CTA = one query sub-tile of <= 256 queries (gridDim.y) x a contiguous share of
 // the launch's blocks (gridDim.x). Per 128-row tile: all 8 warps expand the rows into shared memory, one thread issues WE
 // MMAs into the TMEM accumulator and commits them to an mbarrier while the next tile's words are fetched, then every warp
-// reads its 32 TMEM lanes (warps w and w + 4 split the columns), compares each accumulator with its query's t_q and takes
-// the rare emit path when some lane passes. Two CTAs per SM overlap one's MMA with the other's epilogue.
+// reads its 32 TMEM lanes (warps w and w + 4 split the columns) as packed 16-bit values, compares two accumulators per
+// instruction with their queries' t_q (tc_compare_tile) and takes the rare emit path when some lane passes. Two CTAs per
+// SM overlap one's MMA with the other's epilogue.
 template <int WE>
 __global__ void __launch_bounds__(kThreads, kTcMinBlocksPerSm) k_scan_tc(const __grid_constant__ ScanParams p) {
     constexpr uint32_t KB = 32 * WE;                      // K bytes per row
@@ -116,8 +184,8 @@ __global__ void __launch_bounds__(kThreads, kTcMinBlocksPerSm) k_scan_tc(const _
     const uint32_t NB = tc_round32(p.q_split);            // B rows reserved (same for every CTA of the launch)
     uint8_t* sA = smem_tc;
     uint8_t* sB = sA + kTcRows * KB;
-    int32_t* s_t = reinterpret_cast<int32_t*>(sB + (size_t)NB * KB);
-    uint32_t* s_pq = reinterpret_cast<uint32_t*>(s_t + NB);
+    uint32_t* s_nt = reinterpret_cast<uint32_t*>(sB + (size_t)NB * KB);   // -t_q, packed (tc_compare_tile); NB / 2 used
+    uint32_t* s_pq = s_nt + NB;
     uint64_t* mbar = reinterpret_cast<uint64_t*>(s_pq + NB);
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(mbar + 1);
     uint16_t* s_rank = reinterpret_cast<uint16_t*>(tmem_slot + 2);
@@ -188,10 +256,17 @@ __global__ void __launch_bounds__(kThreads, kTcMinBlocksPerSm) k_scan_tc(const _
     uint32_t item_blocks = p.update_tau ? 1u : p.blocks_per_item;
     for (uint32_t b_lo = my_lo; b_lo < my_hi;) {
         const uint32_t b_hi = min(b_lo + item_blocks, my_hi);
-        __syncthreads();   // the previous item's readers of s_t are done, its candidates are staged
+        __syncthreads();   // the previous item's readers of s_nt are done, its candidates are staged
         if (p.stage_cap) stage_flush(p, s_rank);
-        for (uint32_t q = tid; q < N; q += kThreads)
-            s_t[q] = q < T ? (int32_t)s_hrow[__ldcg(&p.tau[q0 + q])] - (int32_t)s_pq[q] : -0x40000000;   // padding never passes
+        for (uint32_t i = tid; i < N / 2; i += kThreads) {
+            uint32_t w = 0;
+            for (uint32_t hf = 0; hf < 2; hf++) {
+                const uint32_t q = 2 * i + hf;
+                const int32_t nt = q < T ? (int32_t)s_pq[q] - (int32_t)s_hrow[__ldcg(&p.tau[q0 + q])] : 0x4000;   // padding never passes
+                w |= ((uint32_t)nt & 0xffffu) << (16 * hf);
+            }
+            s_nt[i] = w;
+        }
         __syncthreads();
 
         uint32_t v[PER];
@@ -224,27 +299,19 @@ __global__ void __launch_bounds__(kThreads, kTcMinBlocksPerSm) k_scan_tc(const _
             const uint2 blk = p.blocks[ti / kTiles];
             const uint32_t row = blk.y + (ti % kTiles) * kTcRows + lane_base + lane;
             const bool live = row < p.segs[blk.x].n;           // padding rows of the last block never emit
-            for (uint32_t c = col0; c < N / 32; c += 2) {
-                uint32_t acc[32];
-                tmem_ld32(tmem + (lane_base << 16) + c * 32, acc);
-                const int4* tq = reinterpret_cast<const int4*>(s_t + c * 32);
-                int32_t mn = 0x7fffffff;
+            tc_compare_tile(tmem + (lane_base << 16), col0, N / 32, s_nt, live, [&](uint32_t c, const uint32_t (&v)[16]) {
 #pragma unroll
-                for (int j = 0; j < 8; j++) {
-                    const int4 t = tq[j];
-                    mn = min(mn, (int32_t)acc[4 * j] - t.x);
-                    mn = min(mn, (int32_t)acc[4 * j + 1] - t.y);
-                    mn = min(mn, (int32_t)acc[4 * j + 2] - t.z);
-                    mn = min(mn, (int32_t)acc[4 * j + 3] - t.w);
-                }
-                if (__any_sync(0xffffffffu, live && mn <= 0) && live && mn <= 0) {   // rare: re-check the 32 values
+                for (int i = 0; i < 16; i++) {   // unrolled: v stays in registers
+                    const uint32_t nt = s_nt[c * 16 + i];
 #pragma unroll
-                    for (int j = 0; j < 32; j++) {   // unrolled: acc stays in registers
-                        const uint32_t q = c * 32 + j;
-                        if ((int32_t)acc[j] <= s_t[q]) tc_emit(p, q0 + q, tc_hamming((int32_t)acc[j], s_pq[q]), blk.x, row, s_rank);
+                    for (int hf = 0; hf < 2; hf++) {   // sign-extend each half: the exact acc and -t_q
+                        const int32_t acc = hf ? (int32_t)v[i] >> 16 : (int32_t)(int16_t)v[i];
+                        const int32_t neg_t = hf ? (int32_t)nt >> 16 : (int32_t)(int16_t)nt;
+                        const uint32_t q = c * 32 + 2 * i + hf;
+                        if (acc + neg_t <= 0) tc_emit(p, q0 + q, tc_hamming(acc, s_pq[q]), blk.x, row, s_rank);
                     }
                 }
-            }
+            });
             tc_fence_before();
         }
         b_lo = b_hi;
