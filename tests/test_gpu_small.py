@@ -1,8 +1,9 @@
 """
-Small-batch path (csrc/small.cuh: one cooperative launch per search, TMA ring, fused bootstrap and select): every
-request of <= 8 queries takes it. Parity against the oracle for each shape the launch plan distinguishes, and
-equality with the general path (ISX_SMALL_PATH=0 is read once per process, so the general path is exercised here by
-batches of 9+ queries carrying the same queries).
+Small-batch path (csrc/small.cuh: one cooperative launch per search, TMA ring, fused bootstrap and select): by default
+every request of <= 4 queries takes it (ISX_SMALL_MAXQ, at most 8). Parity against the oracle for each shape the launch
+plan distinguishes, and equality with the general path (ISX_SMALL_PATH=0 is read once per process, so the general path
+is exercised here by batches of 5+ queries carrying the same queries). Every compared length, rows on the bound and the
+ISX_SMALL_* switches: tests/test_gpu_scan_edges.py.
 """
 
 import numpy as np

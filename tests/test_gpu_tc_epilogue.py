@@ -35,35 +35,47 @@ def _flip(rng, code, L, nflip):
     return out
 
 
-def bound_case(thr):
+def bound_case(thr, per_length=QUERIES_PER_LENGTH, lengths=tuple(range(1, 33)), row_steps=(0,), n_fill=2048):
     """
-    For every length L = 1..32 bytes, 64 random queries of L bytes and, per query, one row of L bytes exactly on the
-    threshold (h = floor(thr * 8L)) and one a bit past it; plus random rows of every length.
-    -> (keys, codes, lens, queries, qlens, on_rows, past_rows)
+    For every query length L of `lengths`, `per_length` random queries of L bytes (one count for all lengths, or one per
+    length). Per query and per step s of `row_steps`, the row length Lr is the length s places from L in `lengths` (where
+    that exists); one row of Lr bytes lies exactly on the threshold (h = floor(thr * 8m), m = min(L, Lr)) and one a bit
+    past it. A row longer than its query holds 0xFF past the query's length, so that those bytes differ from the query's
+    zero padding. Plus `n_fill` random rows of the lengths.
+    -> (keys, codes, lens, queries, qlens, on_rows, past_rows, owner): owner[i] is the query of on_rows[i] / past_rows[i]
     """
     num, den = thr
     rng = np.random.default_rng(6100 + 10 * num + den)
-    queries, qlens, rows, lens, on_rows, past_rows = [], [], [], [], [], []
-    for L in range(1, 33):
-        hb = num * 8 * L // den
-        for _ in range(QUERIES_PER_LENGTH):
+    counts = [per_length] * len(lengths) if np.isscalar(per_length) else list(per_length)
+    queries, qlens, rows, lens, on_rows, past_rows, owner = [], [], [], [], [], [], []
+    for i, L in enumerate(lengths):
+        for _ in range(counts[i]):
             q = np.zeros(32, dtype=np.uint8)
             q[:L] = rng.integers(0, 256, size=L, dtype=np.uint8)
+            for s in row_steps:
+                if not 0 <= i + s < len(lengths):
+                    continue
+                Lr = lengths[i + s]
+                m = min(L, Lr)
+                hb = num * 8 * m // den
+                for pos, nflip in ((on_rows, hb), (past_rows, hb + 1)):
+                    row = _flip(rng, q, m, nflip)
+                    row[m:Lr] = 0xFF
+                    row[Lr:] = 0
+                    pos.append(len(rows))
+                    rows.append(row)
+                    lens.append(Lr)
+                owner.append(len(queries))
             queries.append(q)
             qlens.append(L)
-            on_rows.append(len(rows))
-            rows.append(_flip(rng, q, L, hb))
-            past_rows.append(len(rows))
-            rows.append(_flip(rng, q, L, hb + 1))
-            lens += [L, L]
-    n_fill = 2048
-    fill_lens = rng.integers(1, 33, size=n_fill).astype(np.uint8)
+    fill_lens = np.asarray(lengths, dtype=np.uint8)[rng.integers(0, len(lengths), size=n_fill)]
     fill = rng.integers(0, 256, size=(n_fill, 32), dtype=np.uint8)
     fill[np.arange(32)[None, :] >= fill_lens[:, None]] = 0
     codes = np.concatenate([np.stack(rows), fill])
     lens = np.concatenate([np.array(lens, dtype=np.uint8), fill_lens])
     keys = synth.make_keys(0, len(lens), 6101 + num)
-    return keys, codes, lens, np.stack(queries), np.array(qlens, dtype=np.uint8), np.array(on_rows), np.array(past_rows)
+    return (keys, codes, lens, np.stack(queries), np.array(qlens, dtype=np.uint8), np.array(on_rows), np.array(past_rows),
+            np.array(owner))
 
 
 def ones_case():
@@ -115,18 +127,28 @@ def _check(case, k, thr=None):
     return (gk, gh, gn, gc), stats
 
 
-@pytest.mark.parametrize("thr", [(1, 8), (3, 10)])
-def test_rows_on_the_bound_every_length(cuda, thr):
-    case = bound_case(thr)
-    keys, on_rows, past_rows = case[0], case[5], case[6]
+def check_bound_rows(case, gk, gc):
+    """Every row planted on the bound is in its query's result, every row one bit past it is not."""
+    keys, on_rows, past_rows, owner = case[0], case[5], case[6], case[7]
+    for on, past, q in zip(on_rows, past_rows, owner):
+        got = set(gk[q, : gc[q]].tolist())
+        assert int(keys[on]) in got, f"query {q}: the row on the bound is missing"
+        assert int(keys[past]) not in got, f"query {q}: the row past the bound is returned"
+
+
+# 64 queries per length: every length tile takes the tensor-core scan; 16: every tile takes the POPC scan (k_scan)
+@pytest.mark.parametrize("thr,per_length", [((1, 8), 64), ((3, 10), 64), ((1, 8), 16), ((3, 10), 16)],
+                         ids=["thr0", "thr1", "thr0-popc", "thr1-popc"])
+def test_rows_on_the_bound_every_length(cuda, thr, per_length):
+    case = bound_case(thr, per_length)
     k = 2048   # above the count of any query (a 1-byte query compares one byte of every row)
     (gk, _, _, gc), stats = _check(case, k, thr)
-    assert stats["issued_popc"] == 0   # only tensor-core launches
+    if per_length >= QUERIES_PER_LENGTH:
+        assert stats["issued_popc"] == 0   # only tensor-core launches
+    else:
+        assert stats["issued_popc"] > 0   # tiles of 16 queries: the POPC scan
     assert (gc < k).all()              # every row within the threshold is in the result
-    for i in range(len(on_rows)):
-        got = set(gk[i, : gc[i]].tolist())
-        assert int(keys[on_rows[i]]) in got, f"query {i}: the row on the bound is missing"
-        assert int(keys[past_rows[i]]) not in got, f"query {i}: the row past the bound is returned"
+    check_bound_rows(case, gk, gc)
 
 
 def test_accumulator_minus_256(cuda):
