@@ -1841,7 +1841,11 @@ int isx_search(isx_store_t* s, const uint8_t* queries, const uint8_t* qlens, siz
         uint32_t H = 2;
         while (H < 2 * k) H <<= 1;
         const size_t smem = (size_t)H * 12 + 16;
-        if (smem + 2048 > (size_t)s->max_smem_optin) return fail(ISX_ELIMIT, "first_of_asset_out supports count <= %u", (uint32_t)(s->max_smem_optin / 24 / 2));
+        if (smem + 2048 > (size_t)s->max_smem_optin) {
+            uint32_t H_max = 2;   // largest table that fits: every count with 2 * count <= H_max is accepted
+            while ((size_t)H_max * 2 * 12 + 16 + 2048 <= (size_t)s->max_smem_optin) H_max <<= 1;
+            return fail(ISX_ELIMIT, "first_of_asset_out supports count <= %u", H_max / 2);
+        }
         if (s->d_stage_codes.ensure(qk)) return ISX_ENOMEM;
         {
             cudaFuncAttributes fa;
