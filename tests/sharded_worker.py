@@ -37,6 +37,11 @@ if args.backend == "nccl":
     perm = np.random.default_rng(7).permutation(q)
     gk2, gh2, gn2, gc2 = (a.copy() for a in searcher.search(np.ascontiguousarray(queries[perm]), np.ascontiguousarray(qlens[perm]), k))
     inv = np.argsort(perm)
+    # 80 queries of every length: every tile has >= 64 queries, so the shared thresholds run through k_scan_tc
+    tc = [synth.make_queries(80, n, 40 + L, 31, lengths=(L,)) for L in synth.STANDARD_LENGTHS]
+    qtc, qltc = np.concatenate([t[0] for t in tc]), np.concatenate([t[1] for t in tc])
+    gktc, ghtc, gntc, gctc = (a.copy() for a in searcher.search(qtc, qltc, k))
+    popc_tc = st.stats()["issued_popc"]
     # third batch: 150K extra rows sharing ONE code -> every rank's candidate buffer overflows for that query and the
     # exact re-scan path runs while thresholds are shared; the merged result must be the 100 smallest keys among the ties
     dup_n = 45_000 * world   # > the candidate buffer (32768) on every rank
@@ -70,7 +75,7 @@ if args.backend == "nccl":
                  shared=s4.shared)
     if rank == 0:
         np.savez(args.out, keys=gk, h=gh, nb=gn, cnt=gc, keys2=gk2[inv], h2=gh2[inv], nb2=gn2[inv], cnt2=gc2[inv], n=n, q=q, k=k,
-                 shared=searcher.shared)
+                 shared=searcher.shared, keys_tc=gktc, h_tc=ghtc, nb_tc=gntc, cnt_tc=gctc, popc_tc=popc_tc)
     dist.barrier()
     dist.destroy_process_group()
 else:

@@ -127,6 +127,12 @@ def test_multi_rank_nccl_search_with_shared_thresholds_equals_oracle(cuda, tmp_p
     # two batches were searched back to back (reset/fence protocol of the shared histograms): both must be exact
     assert_same_topk(d["keys"], d["h"], d["nb"], d["cnt"], keys, rows, h, nb, cnt)
     assert_same_topk(d["keys2"], d["h2"], d["nb2"], d["cnt2"], keys, rows, h, nb, cnt)
+    # >= 64 queries per length: the tensor-core scan with shared thresholds
+    tc = [synth.make_queries(80, n, 40 + L, 31, lengths=(L,)) for L in synth.STANDARD_LENGTHS]
+    qtc, qltc = np.concatenate([t[0] for t in tc]), np.concatenate([t[1] for t in tc])
+    assert int(d["popc_tc"]) == 0, "every tile of the batch was meant to run on the tensor cores"
+    rows_tc, h_tc, nb_tc, cnt_tc = oracle_topk(keys, codes, lens, qtc, qltc, k)
+    assert_same_topk(d["keys_tc"], d["h_tc"], d["nb_tc"], d["cnt_tc"], keys, rows_tc, h_tc, nb_tc, cnt_tc)
     # third batch: mass duplicates -> candidate overflow + exact re-scan on every rank, thresholds still shared
     dd = np.load(str(out).replace(".npz", "_dup.npz"))
     dup_n = int(dd["dup_n"])
